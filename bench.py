@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (our CUDA engine, through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  (the CPU restatement of the reference path)
+  python bench.py ... --dump-outputs DIR                   (also write the last step's outputs as DIR/*.npy)
 
 One "step" = one `pgibbs_sweep!`-equivalent over the observation class: the K-particle row
 moves of every row + the table-update pass (`--sweep all`: over EVERY class in class_order,
@@ -21,6 +22,7 @@ and for `--impl reference`; the measured product path never touches it.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -52,7 +54,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-rows", type=int, default=0, help="--impl reference: rows each process sweeps per step (default per workload)")
     ap.add_argument("--seed", type=int, default=20260924)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the caller received in the last end-to-end step "
+                         "(log-weights and reference slots of the observation rows; with several GPUs, the rows "
+                         "rank 0 owns) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if a.rows <= 0:
         a.rows = {"h1m": 1_000_000, "r10m": 10_000_000, "rents": 50_000, "flights": 2_376}[a.workload]
     if a.particles <= 0:
@@ -219,12 +229,25 @@ class ClockSampler:
                                       stdout=self.f, stderr=subprocess.DEVNULL)
         except Exception:
             self.p = None
+        atexit.register(self._close)      # an exception before stop() must not leave nvidia-smi running
+
+    def _close(self):
+        if self.p and self.p.poll() is None:
+            self.p.terminate()
+            try:
+                self.p.wait(timeout=5)
+            except Exception:
+                self.p.kill()
+        if os.path.exists(self.f.name):
+            self.f.close()
+            os.unlink(self.f.name)
 
     def stop(self, t_begin=None, t_end=None):
         """median SM clock / throttle reasons over the samples taken inside [t_begin, t_end] (time.time());
         nvidia-smi needs ~0.5 s to start, so it is launched long before the timed region"""
         import datetime
         if not self.p:
+            self._close()
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.p.terminate()
         try:
@@ -233,9 +256,11 @@ class ClockSampler:
             self.p.kill()
         self.f.flush()
         self.f.seek(0)
+        lines = self.f.read().strip().splitlines()
+        self._close()
         sm, mx, reasons = [], [], set()
         rows = []
-        for line in self.f.read().strip().splitlines():
+        for line in lines:
             parts = [x.strip() for x in line.split(",")]
             if len(parts) < 9:
                 continue
@@ -268,6 +293,27 @@ def survey_bytes_per_row_particle(model, query, ir, e, nb):
         tot += cands * 4.0 * (f + 1)
         ftot += f
     return tot + 4.0 * ftot + 12.0
+
+
+DUMP_BYTES = 60_000_000      # under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, received, r0, r1, seed, log):
+    """Write the arrays of `received` (one entry per row of [r0, r1)) as float64 .npy files, with
+    `rows.npy` holding the global row indices.  When they do not fit DUMP_BYTES, the same sample of
+    rows, drawn from `seed`, is taken from every array, so runs with the same arguments dump the
+    same rows."""
+    import numpy as np
+    n = r1 - r0
+    keep = max(1, DUMP_BYTES // (8 * (len(received) + 1)))
+    idx = np.arange(n)
+    if n > keep:
+        idx = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), (r0 + idx).astype(np.float64))
+    for name, v in received.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(v)[idx].astype(np.float64))
+    log(f"dumped {len(received) + 1} arrays of {len(idx)} of {n} rows to {out_dir}")
 
 
 def main():
@@ -396,6 +442,7 @@ def main():
     barrier()
     w0 = time.perf_counter()
     h2d = d2h = 0
+    received = {}
     for _ in range(a.steps):
         h2d = e.update_observations(sid_cols, real_cols, r0, r1)
         e.sweep(sweep_cls, a.seed, sweep_idx); sweep_idx += 1
@@ -403,8 +450,10 @@ def main():
         for f in fks:
             k = e.download_assignment_range(cls, f, r0, r1)
             d2h += k.nbytes // 2                                   # device side: int32 slots
+            received[f"assignment_v{f}"] = k
         lw = e.download_logweights_range(cls, r0, r1)
         d2h += lw.nbytes
+        received["logweights"] = lw
     barrier()
     t = torch.tensor([time.perf_counter() - w0, float(h2d), float(d2h)], dtype=torch.float64, device="cuda")
     tsum = t.clone()
@@ -414,6 +463,8 @@ def main():
     e2e_value = n_rows * a.particles * a.steps / float(t[0])
     h2d_total, d2h_total = int(tsum[1]), int(tsum[2])                 # whole job, all ranks
 
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, received, r0, r1, a.seed, log)
     if rank == 0:
         # roofline of the dominant kernel (the block kernel with the larger device time)
         peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")

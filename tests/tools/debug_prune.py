@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 from pclean_b200.host_fixture import model as M
 from tests.test_engine_parity import _setup_synth
 cfg = M.InferenceConfig(1, 20)
